@@ -10,6 +10,9 @@ long/long packets (spectrum [S][P][2][1024] f32, device-resident, > L2), through
 lwb_decode_chains (fused kernel k_long).  `value` = channel-samples per second over all ranks,
 timed with CUDA events on the library's stream, max over ranks.  `e2e` = the same call with HOST
 (pinned) buffers: H2D of the spectrum and D2H of the PCM inside the timed region.
+
+--dump-outputs DIR writes what the last timed step returned (inputs are seeded: the same arguments give the same
+inputs), so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -26,6 +29,20 @@ sys.path.insert(0, ROOT)
 
 N2 = 1024
 ALG_BYTES_PER_SAMPLE = 8          # 4 B spectrum read + 4 B f32 PCM write (SURVEY.md section 8d)
+DUMP_PCM_BYTES = 48 << 20         # --dump-outputs: PCM sample size cap (the whole dump stays under 64 MB)
+DUMP_SEED = 2024
+
+
+def timed_outputs(pcm, batch):
+    """--dump-outputs: what a caller of the timed step receives after its last run -- the PCM of a fixed, seeded
+    sample of the streams (all of them when they fit DUMP_PCM_BYTES) and every chain's result fields."""
+    S = pcm.shape[0]
+    k = min(S, DUMP_PCM_BYTES // (pcm[0].numel() * pcm.element_size()))
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(S, k, replace=False))
+    res = [(c.n_samples, c.packets_done, c.status) for c in batch.collect()]
+    return {"pcm": pcm[idx.tolist()].cpu().numpy(),                   # [k][channels][packets * 1024] f32
+            "pcm_streams": idx.astype(np.float64),                     # the sampled stream indices
+            "chain_results": np.array(res, np.float64)}                # [streams][n_samples, packets_done, status]
 
 
 def peaks():
@@ -171,7 +188,17 @@ def main():
     ap.add_argument("--mixed-streams", type=int, default=2048,
                     help="streams per GPU of the mixed short/long measurement (0: skip)")
     ap.add_argument("--sustained-sec", type=float, default=1.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs of the last one as DIR/<name>.npy (pcm: a seeded "
+                         "sample of the streams; pcm_streams: their indices; chain_results: per-chain n_samples, "
+                         "packets_done, status)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path; the reference arm has no outputs to dump")
+    if args.dump_outputs and 2 * args.packets * N2 * 4 > DUMP_PCM_BYTES:
+        ap.error(f"--dump-outputs: one stream's PCM exceeds {DUMP_PCM_BYTES >> 20} MB; use fewer --packets")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -249,6 +276,7 @@ def main():
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     launches = ctx.launch_count - l0
+    dumped = timed_outputs(pcm, batch) if args.dump_outputs and rank == 0 else {}
     # The timed region lasts a few milliseconds (a burst, far below nvidia-smi's sampling period).  The same step is
     # then repeated back to back for >= --sustained-sec, timed the same way: that is the sustained value (power
     # capped clocks), and the window the clock / throttle samples are taken in.
@@ -481,6 +509,10 @@ def main():
                                               f"{sec:.2f} s wall on {threads} threads ({sec * threads:.0f} core-s); "
                                               "lewton-equivalent C restatement (oracle/), the crate itself is Rust"}
         os.write(json_fd, (json.dumps(line) + "\n").encode())
+    if dumped:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.destroy_process_group()
     return 0
