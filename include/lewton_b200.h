@@ -70,6 +70,8 @@ const char *lwb_last_error(const lwb_ctx *ctx);
 void *lwb_ctx_cuda_stream(lwb_ctx *ctx);
 /* kernels launched by this ctx since creation (bench.py's gpu_launches) */
 uint64_t lwb_ctx_launch_count(const lwb_ctx *ctx);
+/* of those, launches of the fused long-block kernels (k_long, k_long_s): tells the fused path from the chain kernel */
+uint64_t lwb_ctx_long_launch_count(const lwb_ctx *ctx);
 /* pinned host memory for the host-buffer entry points (optional; plain malloc'd memory works, slower) */
 void *lwb_host_alloc(size_t bytes);
 void lwb_host_free(void *p);

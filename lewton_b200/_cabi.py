@@ -93,6 +93,7 @@ SYMBOLS = {
     "lwb_last_error": (C.c_char_p, [vp]),
     "lwb_ctx_cuda_stream": (vp, [vp]),
     "lwb_ctx_launch_count": (C.c_uint64, [vp]),
+    "lwb_ctx_long_launch_count": (C.c_uint64, [vp]),
     "lwb_host_alloc": (vp, [C.c_size_t]),
     "lwb_bind_host_to_device": (C.c_int, [C.c_int]),
     "lwb_host_free": (None, [vp]),

@@ -64,6 +64,11 @@ class Context:
     def launch_count(self):
         return cabi.lib().lwb_ctx_launch_count(self._h)
 
+    @property
+    def long_launch_count(self):
+        """Launches of the fused long-block kernels (k_long, k_long_s) among launch_count."""
+        return cabi.lib().lwb_ctx_long_launch_count(self._h)
+
     def device_alloc(self, nbytes):
         p = C.c_void_p()
         self.check(cabi.lib().lwb_device_alloc(self._h, nbytes, C.byref(p)))

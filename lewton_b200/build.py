@@ -36,13 +36,14 @@ def check_no_fma(so=SO):
 
 
 def hot_kernel_registers(log):
-    """Registers per thread of k_long<float> / k_long<int16_t> from ptxas -v output.  The headline kernel is bound by
-    per-warp latency and touchy about its allocation: at 254-255 registers (two more live values, or a changed helper
-    template that only its sibling k_long_s uses) it lost 3-4 % (A/B on one box, DESIGN.md 4.4); 250 / 252 is the
-    allocation the measured numbers belong to."""
+    """Registers per thread of every k_long<OutT, CS> instantiation (CS = 1 planar, 2..8 interleaved) from ptxas -v
+    output.  The headline kernel is bound by per-warp latency and touchy about its allocation: at 254-255 registers
+    (two more live values, or a changed helper template that only its sibling k_long_s uses) it lost 3-4 % (A/B on one
+    box, DESIGN.md 4.4); 250 / 252 is the allocation the measured planar numbers belong to, 253-254 the one of the
+    interleaved instantiations (DESIGN.md 4.7)."""
     regs = {}
-    for m in re.finditer(r"Compiling entry function '(_ZN3lwb6k_longI([fs])EE[^']*)'.*?Used (\d+) registers", log, re.S):
-        regs["k_long<float>" if m.group(2) == "f" else "k_long<int16_t>"] = int(m.group(3))
+    for m in re.finditer(r"Compiling entry function '(_ZN3lwb6k_longI([fs])Li(\d+)EE[^']*)'.*?Used (\d+) registers", log, re.S):
+        regs[f"k_long<{'float' if m.group(2) == 'f' else 'int16_t'}, {m.group(3)}>"] = int(m.group(4))
     return regs
 
 
@@ -57,9 +58,11 @@ def build(force=False, verbose=False):
         if r.returncode:
             raise RuntimeError("nvcc build of liblewton_b200.so failed")
         regs = hot_kernel_registers(r.stdout + r.stderr)
-        if any(v > 252 for v in regs.values()):
-            print(f"lewton_b200 build: WARNING: {regs} -- k_long above 252 registers has measured 3-4 % slower; "
-                  "look at what changed in kernel_long.cuh's shared helpers")
+        if len(regs) != 16:
+            print(f"lewton_b200 build: WARNING: found {len(regs)} of the 16 k_long instantiations in the ptxas log")
+        if any(v > (252 if k.endswith(", 1>") else 254) for k, v in regs.items()):
+            print(f"lewton_b200 build: WARNING: {regs} -- k_long above 252 registers (planar) / 254 (interleaved) has "
+                  "measured 3-4 % slower; look at what changed in kernel_long.cuh's shared helpers")
         n = check_no_fma()
         if n:
             os.remove(SO)

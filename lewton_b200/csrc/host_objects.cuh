@@ -43,6 +43,7 @@ struct lwb_ctx {
     uint64_t state_gen = 1;        // bumped whenever any stream's (has, len) changes: plans key on it
     std::string err;
     uint64_t launches = 0;
+    uint64_t long_launches = 0;    // of which k_long / k_long_s
     std::deque<CachedTables> tables;       // (deque: setups hold copies of dt, growth never moves an entry)
     // grow-only device arenas
     DevBuf coeffs, dense, pcm, spec, segtab, vqoff, vqrec, magic, x, desc, kinds, ys, chains, ticket, cdesc, cbytes;
@@ -87,6 +88,7 @@ struct lwb_plan {
     uint32_t n_groups = 0;
     const float *pack = nullptr;
     bool i16 = false;
+    int step = 1;                  // k_long's PCM step: 1 planar, the channel count interleaved
     // residue entry: the front-stage descriptors (one DevPacket per packet).  They depend only on the captured
     // chain / mode arrays, never on stream state, so they stay valid for the plan's lifetime.
     bool pro_captured = false, pro_fast = false;

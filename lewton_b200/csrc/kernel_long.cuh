@@ -625,7 +625,7 @@ __device__ __forceinline__ void st_pcm(int16_t *p, float v) { __stcs(reinterpret
 // run -- its previous right half comes from the stream state (staged in shared memory by TMA
 // while the run's first tile was in flight) if has_prev, else nothing is emitted.  Streaming
 // stores: PCM is written once and never read back by this kernel.
-template <int NB, bool FIRST, typename OutT, typename RC = RunCur>
+template <int NB, bool FIRST, typename OutT, typename RC = RunCur, int CS = 1>
 __device__ __forceinline__ void out_stage(const TwMix &tw, int lane, const V O[NB][8], const V E[NB][8], V pe[NB][8],
                                           const RC cur[NB], OutT *out[NB], const float *s_state)
 {
@@ -656,13 +656,14 @@ __device__ __forceinline__ void out_stage(const TwMix &tw, int lane, const V O[N
             pe[b][j] = pev;
             if (emit) {
                 // m = r64 + lane (or + 63 - lane); 1023 - m = 960 - r64 + 63 - lane (or + lane)
-                OutT *o_lo = out[b] + lane, *o_hi = out[b] + 63 - lane;
+                // (CS: samples between consecutive PCM elements of one channel -- 1 planar, C interleaved)
+                OutT *o_lo = out[b] + lane * CS, *o_hi = out[b] + 63 * CS - lane * CS;
                 if (nat) {
-                    st_pcm(o_lo + r64, lo.x); st_pcm(o_hi + r64, lo.y);
-                    st_pcm(o_hi + 960 - r64, hi.x); st_pcm(o_lo + 960 - r64, hi.y);
+                    st_pcm(o_lo + r64 * CS, lo.x); st_pcm(o_hi + r64 * CS, lo.y);
+                    st_pcm(o_hi + 960 * CS - r64 * CS, hi.x); st_pcm(o_lo + 960 * CS - r64 * CS, hi.y);
                 } else {
-                    st_pcm(o_hi + r64, lo.x); st_pcm(o_lo + r64, lo.y);
-                    st_pcm(o_lo + 960 - r64, hi.x); st_pcm(o_hi + 960 - r64, hi.y);
+                    st_pcm(o_hi + r64 * CS, lo.x); st_pcm(o_lo + r64 * CS, lo.y);
+                    st_pcm(o_lo + 960 * CS - r64 * CS, hi.x); st_pcm(o_hi + 960 * CS - r64 * CS, hi.y);
                 }
             }
         }
@@ -685,7 +686,7 @@ __device__ __forceinline__ float lds_f32(uint32_t addr)
 // at w_s (through __ldg from global memory the four products of a lane each waited for an L2 round trip: 3.4 % of
 // k_long_s's stall samples on the 6-channel config)
 // LS: ls as a compile-time constant (0: use the argument) -- with it every position test below folds per slot.
-template <int NB, typename OutT, typename RC = RunCur, bool EXPORT = false, int LS = 0>
+template <int NB, typename OutT, typename RC = RunCur, bool EXPORT = false, int LS = 0, int CS = 1>
 __device__ __forceinline__ void out_first_short(const TwMix &tw, int lane, const V O[NB][8], const V E[NB][8], V pe[NB][8],
                                                 const RC cur[NB], OutT *out[NB], const float *s_state,
                                                 const float *__restrict__ w, int ls_arg, uint32_t w_s = 0)
@@ -716,7 +717,7 @@ __device__ __forceinline__ void out_first_short(const TwMix &tw, int lane, const
                     const int i = m - ls;                                      // < pl / 2
                     const float cw = __fmul_rn(po, (EXPORT ? lds_f32(w_s + 4u * (uint32_t)i) : __ldg(w + i)));
                     if (exported) cur[b].state[i] = cw;
-                    else st_pcm(out[b] + i, __fadd_rn(cw, __fmul_rn(prev[i], (EXPORT ? lds_f32(w_s + 4u * (uint32_t)(pl - 1 - i)) : __ldg(w + pl - 1 - i)))));
+                    else st_pcm(out[b] + i * CS, __fadd_rn(cw, __fmul_rn(prev[i], (EXPORT ? lds_f32(w_s + 4u * (uint32_t)(pl - 1 - i)) : __ldg(w + pl - 1 - i)))));
                 }
                 const int i = kLongN2 - 1 - m - ls;                            // >= pl / 2
                 float v = -po;
@@ -725,7 +726,7 @@ __device__ __forceinline__ void out_first_short(const TwMix &tw, int lane, const
                     if (exported) { cur[b].state[i] = v; continue; }
                     v = __fadd_rn(v, __fmul_rn(prev[i], (EXPORT ? lds_f32(w_s + 4u * (uint32_t)(pl - 1 - i)) : __ldg(w + pl - 1 - i))));
                 }
-                st_pcm(out[b] + i, v);
+                st_pcm(out[b] + i * CS, v);
             }
         }
     }
@@ -741,7 +742,9 @@ __device__ __forceinline__ void out_first_short(const TwMix &tw, int lane, const
 //     a packet later; its descriptors then arrive by TMA into shared memory;
 //   * the stream state a run overlaps with (has_prev) arrives by TMA into a per-warp state tile
 //     while the run's first spectrum tile is in flight.
-template <typename OutT>
+// CS: PCM step of a channel (1: planar; C: interleaved, one instantiation per channel count so that every store
+// offset stays an immediate and the planar instantiations keep their code)
+template <typename OutT, int CS = 1>
 __global__ void __launch_bounds__(kLongWarps * 32, 1)
 k_long(const LongRun *__restrict__ runs, uint32_t n_groups, const float *__restrict__ pack,
        unsigned int *__restrict__ ticket, const float *__restrict__ w_short, int ls)
@@ -960,19 +963,19 @@ k_long(const LongRun *__restrict__ runs, uint32_t n_groups, const float *__restr
             }
             phase_c_fft<NB>(tw, O, E);
             if (p > 0) {
-                out_stage<NB, false, OutT>(tw, lane, O, E, pe, cur, out, s_state);
+                out_stage<NB, false, OutT, RunCur, CS>(tw, lane, O, E, pe, cur, out, s_state);
             } else {
                 mbar_wait(bar_state, (phase_bits >> 30) & 1u);      // armed once per group
                 phase_bits ^= 1u << 30;
                 if (NB == 1 && (cur[0].flags & 8u))
-                    out_first_short<NB, OutT>(tw, lane, O, E, pe, cur, out, s_state, w_short, ls);
+                    out_first_short<NB, OutT, RunCur, false, 0, CS>(tw, lane, O, E, pe, cur, out, s_state, w_short, ls);
                 else
-                    out_stage<NB, true, OutT>(tw, lane, O, E, pe, cur, out, s_state);
+                    out_stage<NB, true, OutT, RunCur, CS>(tw, lane, O, E, pe, cur, out, s_state);
                 __syncwarp();                                       // state tile consumed
             }
 #pragma unroll
             for (int b = 0; b < NB; b++)
-                if (p > 0 || (cur[b].flags & 1u)) out[b] += (p == 0 && (cur[b].flags & 8u)) ? kLongN2 - ls : kLongN2;
+                if (p > 0 || (cur[b].flags & 1u)) out[b] += ((p == 0 && (cur[b].flags & 8u)) ? kLongN2 - ls : kLongN2) * CS;
             // the state tile is free after packet 0: request the next group's state rows as soon as
             // its descriptors are known
             if (lane == 0 && nx_stage == 2 && !nx_state_issued) {
@@ -1002,7 +1005,7 @@ k_long(const LongRun *__restrict__ runs, uint32_t n_groups, const float *__restr
                         const float v = ((j & 1) != 0) == (h == 0) ? pe[b][j].x : pe[b][j].y;
                         const int m = r64 + (h ? 63 - lane : lane);          // x[1024 + m] = x[2047 - m] = v
                         if (m < ls) {
-                            if (emitted) st_pcm(out[b] + m, v);
+                            if (emitted) st_pcm(out[b] + m * CS, v);
                         } else if (keep && m < kLongN2 - ls) {      // the pl = 1024 - 2 ls samples the short block overlaps with
                             cur[b].state[m - ls] = v;
                             cur[b].state[kLongN2 - 1 - ls - m] = v;
@@ -1350,23 +1353,39 @@ inline int long_launch_static(cudaStream_t stream, const LongRun *d_runs, uint32
     return cudaGetLastError() != cudaSuccess;
 }
 
+// The k_long instantiations: planar (CS = 1) and interleaved for 2..8 channels, f32 and i16.
+#define LWB_LONG_STEPS(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8)
+
 inline void long_kernel_configure()
 {
-    cudaFuncSetAttribute(k_long<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytes);
-    cudaFuncSetAttribute(k_long<int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytes);
+#define LWB_LONG_CONF(CS)                                                                                      \
+    cudaFuncSetAttribute(k_long<float, CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytes); \
+    cudaFuncSetAttribute(k_long<int16_t, CS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytes);
+    LWB_LONG_STEPS(LWB_LONG_CONF)
+#undef LWB_LONG_CONF
     cudaFuncSetAttribute(k_long_s<float, kLongLs256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytesS);
     cudaFuncSetAttribute(k_long_s<int16_t, kLongLs256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLongSmemBytesS);
 }
 
 // d_runs: n_groups * kLongNB descriptors.  Returns 0 on success; `ticket` must point at a zeroed
-// device word no other launch in flight uses.
+// device word no other launch in flight uses.  step: PCM elements between consecutive samples of
+// one channel -- 1 for planar output, the channel count (2..8) for interleaved output.
 inline int long_launch(cudaStream_t stream, const LongRun *d_runs, uint32_t n_groups, const float *d_pack,
-                       unsigned int *ticket, int sm_count, bool i16_out, const float *d_w_short = nullptr, int ls = 0)
+                       unsigned int *ticket, int sm_count, bool i16_out, const float *d_w_short = nullptr, int ls = 0, int step = 1)
 {
     const uint32_t want = (n_groups + kLongWarps - 1) / kLongWarps;
     const uint32_t grid = want < (uint32_t)sm_count ? want : (uint32_t)sm_count;
-    if (i16_out) k_long<int16_t><<<grid, kLongWarps * 32, kLongSmemBytes, stream>>>(d_runs, n_groups, d_pack, ticket, d_w_short, ls);
-    else k_long<float><<<grid, kLongWarps * 32, kLongSmemBytes, stream>>>(d_runs, n_groups, d_pack, ticket, d_w_short, ls);
+    switch (step) {
+#define LWB_LONG_CASE(CS)                                                                                                          \
+    case CS:                                                                                                                       \
+        if (i16_out) k_long<int16_t, CS><<<grid, kLongWarps * 32, kLongSmemBytes, stream>>>(d_runs, n_groups, d_pack, ticket, d_w_short, ls); \
+        else k_long<float, CS><<<grid, kLongWarps * 32, kLongSmemBytes, stream>>>(d_runs, n_groups, d_pack, ticket, d_w_short, ls);          \
+        break;
+        LWB_LONG_STEPS(LWB_LONG_CASE)
+#undef LWB_LONG_CASE
+    default:
+        return 1;
+    }
     return cudaGetLastError() != cudaSuccess;
 }
 #endif  // __CUDACC__

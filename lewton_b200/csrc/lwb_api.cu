@@ -122,6 +122,7 @@ extern "C" int lwb_ctx_synchronize(lwb_ctx *ctx)
 extern "C" const char *lwb_last_error(const lwb_ctx *ctx) { return ctx ? ctx->err.c_str() : "no context"; }
 extern "C" void *lwb_ctx_cuda_stream(lwb_ctx *ctx) { return ctx ? (void *)ctx->stream : nullptr; }
 extern "C" uint64_t lwb_ctx_launch_count(const lwb_ctx *ctx) { return ctx ? ctx->launches : 0; }
+extern "C" uint64_t lwb_ctx_long_launch_count(const lwb_ctx *ctx) { return ctx ? ctx->long_launches : 0; }
 
 extern "C" void *lwb_host_alloc(size_t bytes)
 {
@@ -715,9 +716,10 @@ extern "C" int lwb_plan_execute(lwb_plan *p)
         if (ctx->ticket_next % kTicketPool == 0)
             CU(ctx, cudaMemsetAsync(ctx->ticket.p, 0, kTicketPool * sizeof(unsigned int), ctx->stream));
         unsigned int *ticket = (unsigned int *)ctx->ticket.p + (ctx->ticket_next++ % kTicketPool);
-        if (long_launch(ctx->stream, (const LongRun *)p->runs.p, p->n_groups, p->pack, ticket, ctx->sm_count, p->i16))
+        if (long_launch(ctx->stream, (const LongRun *)p->runs.p, p->n_groups, p->pack, ticket, ctx->sm_count, p->i16, nullptr, 0, p->step))
             return fail(ctx, LWB_ERR_CUDA, "long kernel launch", cudaGetLastError());
         ctx->launches++;
+        ctx->long_launches++;
         return LWB_OK;
     }
     if (p->mixed_captured && p->gen == ctx->state_gen && !getenv("LWB_FORCE_GENERIC")) {

@@ -82,6 +82,7 @@ static int mixed_launch_rounds(lwb_ctx *ctx, const MixLaunch &ml, const std::vec
                         : long_launch(sm, (const LongRun *)ml.db + rd.r0, (uint32_t)rd.nr, ml.pack, ticket, ctx->sm_count, ml.i16, ml.w_short, ml.ls))
                 return fail(ctx, LWB_ERR_CUDA, "long kernel launch", cudaGetLastError());
             ctx->launches++;
+            ctx->long_launches++;
         }
         if (rd.ns) {
             if (short_launch(sm, (const ShortRun *)(ml.db + ml.off_sr) + rd.s0, (uint32_t)rd.ns, ml.spack, ctx->sm_count, ml.i16))

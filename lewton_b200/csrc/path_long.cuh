@@ -3,7 +3,8 @@
 #pragma once
 
 // ---------------------------------------------------------------------------------------------
-// Fused path (kernel_long.cuh).  Eligible batches: spectrum entry, planar f32 out, every packet a
+// Fused path (kernel_long.cuh).  Eligible batches: spectrum entry, f32 or i16 out (planar, or interleaved with one
+// channel count of at most 8 per batch), every packet a
 // long block of blocksize 2^11 with long neighbours, every stream either empty or holding a
 // 1024-sample right half.  Planned directly from the chain list in O(chains + mode bytes) -- at
 // 0.8 G blocks/s per GPU a per-packet host plan would be the bottleneck.
@@ -34,39 +35,67 @@ static int acquire_staging(lwb_ctx *ctx, size_t bytes, Staging **out)
     return LWB_OK;
 }
 
+// Whether k_long takes the batch's interleaved output at all (read once per call).  Not with LWB_NO_ITL set, and not
+// for host-memory batches: their sliced H2D / kernel / D2H pipeline measured slower than the chain kernel's single
+// pass for interleaved i16 residue batches (DESIGN 4.7), so those keep the chain kernel.
+static bool long_takes_itl(const lwb_batch_io *io)
+{
+    return io->memory == LWB_MEM_DEVICE && !getenv("LWB_NO_ITL");
+}
+
+// PCM step of a channel on the fused kernels: 1 for planar output, C for interleaved output (k_long is instantiated
+// for C <= 8; mono interleaved is the planar layout).  0: the batch's format stays off the fused kernels (interleaved
+// output with more than 8 channels, or !itl_ok): the chain kernel writes it, as before k_long took interleaved output.
+static unsigned long_step(int fmt, unsigned C, bool itl_ok)
+{
+    if (is_planar(fmt)) return 1;
+    if (C > 8 || !itl_ok) return 0;
+    return C;
+}
+
+// One past the last PCM element a chain of C channels writes.
+static uint64_t pcm_end(const lwb_chain *c, unsigned C, bool planar, uint64_t n_samples)
+{
+    return c->out_offset + (planar ? (uint64_t)(C - 1) * c->out_stride + n_samples : n_samples * C);
+}
+
 // Appends the runs of one chain.  A chain (one channel of one stream) is cut into several runs
 // when there are too few chains to fill the machine; every run after the first re-transforms the
 // packet before its first one as a primer (its right half is all the run needs), which keeps
 // runs independent at the cost of one extra IMDCT per cut.
+// Planar output (step 1): a channel's runs one after the other.  Interleaved output (step C): cut by cut, the C runs
+// that write one stretch of frames next to each other, so that the warps drawing them fill the same PCM lines at
+// about the same time.
 static void long_runs_of(const LongItem &it, size_t cuts, const float *coeffs, uint64_t coeff_base, char *pcm,
-                         uint64_t pcm_base, size_t esz, LongRun *&w)
+                         uint64_t pcm_base, size_t esz, unsigned step, LongRun *&w)
 {
     const lwb_stream *s = it.c->stream;
     const lwb_setup *su = s->setup;
     const unsigned C = su->channels;
     const size_t P = it.P;
-    for (unsigned ch = 0; ch < C; ch++) {
+    const bool itl = step != 1;
+    for (size_t q = 0; q < (size_t)C * cuts; q++) {
+        const unsigned ch = (unsigned)(itl ? q % C : q / cuts);
+        const size_t k = itl ? q / C : q % cuts;
         const float *in0 = coeffs + (it.c->coeff_offset - coeff_base) + (size_t)ch * kLongN2;
-        char *out0 = pcm + ((it.c->out_offset - pcm_base) + (size_t)ch * it.c->out_stride) * esz;
-        for (size_t k = 0; k < cuts; k++) {
-            const size_t p0 = P * k / cuts, p1 = P * (k + 1) / cuts;   // this run emits packets [p0, p1)
-            LongRun &r = *w++;
-            std::memset(&r, 0, sizeof(r));
-            r.in_stride = (uint32_t)(C * kLongN2);
-            r.state = s->d_state + (size_t)ch * state_stride(su);
-            r.write_state = (k + 1 == cuts);
-            if (k == 0) {
-                r.in = in0;
-                r.n_packets = (uint32_t)(p1 - p0);
-                r.has_prev = it.has_prev;
-                r.out = out0;
-            } else {
-                r.in = in0 + (p0 - 1) * (size_t)r.in_stride;           // primer = packet p0 - 1
-                r.n_packets = (uint32_t)(p1 - p0 + 1);
-                r.has_prev = 0;
-                // samples emitted before packet p0: packets 0..p0-1, minus the first if no state
-                r.out = out0 + (size_t)(p0 - (it.has_prev ? 0 : 1)) * kLongN2 * esz;
-            }
+        char *out0 = pcm + ((it.c->out_offset - pcm_base) + (itl ? (size_t)ch : (size_t)ch * it.c->out_stride)) * esz;
+        const size_t p0 = P * k / cuts, p1 = P * (k + 1) / cuts;   // this run emits packets [p0, p1)
+        LongRun &r = *w++;
+        std::memset(&r, 0, sizeof(r));
+        r.in_stride = (uint32_t)(C * kLongN2);
+        r.state = s->d_state + (size_t)ch * state_stride(su);
+        r.write_state = (k + 1 == cuts);
+        if (k == 0) {
+            r.in = in0;
+            r.n_packets = (uint32_t)(p1 - p0);
+            r.has_prev = it.has_prev;
+            r.out = out0;
+        } else {
+            r.in = in0 + (p0 - 1) * (size_t)r.in_stride;           // primer = packet p0 - 1
+            r.n_packets = (uint32_t)(p1 - p0 + 1);
+            r.has_prev = 0;
+            // samples emitted before packet p0: packets 0..p0-1, minus the first if no state
+            r.out = out0 + (size_t)(p0 - (it.has_prev ? 0 : 1)) * kLongN2 * step * esz;
         }
     }
 }
@@ -75,7 +104,8 @@ static void long_runs_of(const LongItem &it, size_t cuts, const float *coeffs, u
 // holding a 1024-sample right half, arenas aligned: what the fused kernel takes.
 static bool batch_is_uniform_long(lwb_ctx *ctx, const lwb_chain *chains, size_t n_chains, const lwb_batch_io *io)
 {
-    if (io->out_format != LWB_OUT_F32_PLANAR && io->out_format != LWB_OUT_I16_PLANAR) return false;
+    const bool planar = is_planar(io->out_format);
+    const bool itl_ok = long_takes_itl(io);
     const float *pack = nullptr;
     for (size_t i = 0; i < n_chains; i++) {
         const lwb_chain *c = &chains[i];
@@ -85,7 +115,8 @@ static bool batch_is_uniform_long(lwb_ctx *ctx, const lwb_chain *chains, size_t 
         if (su->bs1 != kLongBs || !su->host.tab[1].pack) return false;
         if (pack && pack != su->host.tab[1].pack) return false;
         pack = su->host.tab[1].pack;
-        if ((c->out_offset & 3) || (c->out_stride & 3) || (c->coeff_offset & 3)) return false;
+        if (!long_step(io->out_format, su->channels, itl_ok)) return false;
+        if ((c->out_offset & 3) || (planar && (c->out_stride & 3)) || (c->coeff_offset & 3)) return false;
         if (s->has && s->plen != (uint32_t)kLongN2) return false;
         for (uint32_t k = 0; k < c->n_packets; k++) {
             const uint8_t m = c->mode_numbers[k];
@@ -116,14 +147,16 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
     const uint64_t gen_at_entry = ctx->state_gen;
     if (plan) plan->captured = false;
     if (!spectrum_dev && io->entry != LWB_ENTRY_SPECTRUM) return LWB_OK;
-    if (io->out_format != LWB_OUT_F32_PLANAR && io->out_format != LWB_OUT_I16_PLANAR) return LWB_OK;
     if (getenv("LWB_FORCE_GENERIC")) return LWB_OK;
-    const bool i16 = io->out_format == LWB_OUT_I16_PLANAR;
-    const size_t esz = i16 ? 2 : 4;
+    const bool planar = is_planar(io->out_format);
+    const bool i16 = io->out_format == LWB_OUT_I16_PLANAR || io->out_format == LWB_OUT_I16_INTERLEAVED;
+    const size_t esz = elem_size(io->out_format);
     std::vector<LongItem> items;
     items.reserve(n_chains);
     const float *pack = nullptr;
     size_t chan_chains = 0;
+    unsigned step = 0;                 // interleaved: one channel count per launch, it is the kernel's store step
+    const bool itl_ok = long_takes_itl(io);
     for (size_t i = 0; i < n_chains; i++) {
         lwb_chain *c = &chains[i];
         if (!c->stream || c->stream->ctx != ctx || (c->n_packets && !c->mode_numbers)) return LWB_OK;   // generic path reports it
@@ -132,7 +165,10 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
         if (su->bs1 != kLongBs || !su->host.tab[1].pack) return LWB_OK;
         if (pack && pack != su->host.tab[1].pack) return LWB_OK;          // one twiddle pack per launch
         pack = su->host.tab[1].pack;
-        if ((c->out_offset & 3) || (c->out_stride & 3) || (c->coeff_offset & 3)) return LWB_OK;
+        const unsigned cs = long_step(io->out_format, su->channels, itl_ok);
+        if (!cs || (step && cs != step)) return LWB_OK;
+        step = cs;
+        if ((c->out_offset & 3) || (planar && (c->out_stride & 3)) || (c->coeff_offset & 3)) return LWB_OK;
         if (s->has && s->plen != (uint32_t)kLongN2) return LWB_OK;
         const uint32_t P = c->n_packets;
         for (uint32_t k = 0; k < P; k++) {
@@ -158,11 +194,11 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
         c->packets_done = it.P;
         c->n_samples = it.P ? (uint32_t)((it.P - (it.has_prev ? 0 : 1)) * kLongN2) : 0;
         if (!it.P) continue;
-        if (c->out_stride < c->n_samples) return fail(ctx, LWB_ERR_BUFFER, "chain: out_stride smaller than the samples produced");
+        if (planar && c->out_stride < c->n_samples) return fail(ctx, LWB_ERR_BUFFER, "chain: out_stride smaller than the samples produced");
         c_lo = std::min(c_lo, c->coeff_offset);
         c_hi = std::max(c_hi, c->coeff_offset + (uint64_t)it.P * C * kLongN2);
         o_lo = std::min(o_lo, c->out_offset);
-        o_hi = std::max(o_hi, c->out_offset + (uint64_t)(C - 1) * c->out_stride + c->n_samples);
+        o_hi = std::max(o_hi, pcm_end(c, C, planar, c->n_samples));
     }
     if (!chan_chains) return LWB_OK;
     const size_t warp_slots = (size_t)ctx->sm_count * kLongWarps * kLongNB;
@@ -259,13 +295,13 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
         }
         for (size_t i = i0; i < i1; i++) {
             if (!items[i].P) continue;
-            long_runs_of(items[i], cuts[i], d_coeffs, cbase, d_pcm, obase, esz, gen);
+            long_runs_of(items[i], cuts[i], d_coeffs, cbase, d_pcm, obase, esz, step, gen);
             const lwb_chain *c = items[i].c;
             const unsigned C = c->stream->setup->channels;
             kc_lo = std::min(kc_lo, c->coeff_offset);
             kc_hi = std::max(kc_hi, c->coeff_offset + (uint64_t)items[i].P * C * kLongN2);
             ko_lo = std::min(ko_lo, c->out_offset);
-            ko_hi = std::max(ko_hi, c->out_offset + (uint64_t)(C - 1) * c->out_stride + c->n_samples);
+            ko_hi = std::max(ko_hi, pcm_end(c, C, planar, c->n_samples));
         }
         if (!chunk_runs) continue;
         if (kLongNB == 1) {
@@ -321,9 +357,10 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
         if (ctx->ticket_next % kTicketPool == 0)
             CU(ctx, cudaMemsetAsync(ctx->ticket.p, 0, kTicketPool * sizeof(unsigned int), ctx->stream));
         unsigned int *ticket = (unsigned int *)ctx->ticket.p + (ctx->ticket_next++ % kTicketPool);
-        if (long_launch(ctx->stream, d_runs_base + cp.r0, (uint32_t)(cp.nr / kLongNB), pack, ticket, ctx->sm_count, i16))
+        if (long_launch(ctx->stream, d_runs_base + cp.r0, (uint32_t)(cp.nr / kLongNB), pack, ticket, ctx->sm_count, i16, nullptr, 0, (int)step))
             return fail(ctx, LWB_ERR_CUDA, "long kernel launch", cudaGetLastError());
         ctx->launches++;
+        ctx->long_launches++;
         if (host && cp.ko_hi > cp.ko_lo) {
             const size_t evk = slice.active ? (size_t)slice.ev_slot : k;
             CU(ctx, cudaEventRecord(ctx->ev_done[evk], ctx->stream));
@@ -339,6 +376,7 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
         plan->n_groups = (uint32_t)(cplan[0].nr / kLongNB);
         plan->pack = pack;
         plan->i16 = i16;
+        plan->step = (int)step;
     }
     if (host && !slice.active) {
         CU(ctx, cudaStreamSynchronize(ctx->copy_out));
@@ -353,11 +391,12 @@ static int try_long(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, const lwb_
 // kernel takes) -- decided from the generic plan.
 static bool plan_is_long(const std::vector<PlanChain> &plan, const lwb_batch_io *io)
 {
-    if (io->out_format != LWB_OUT_F32_PLANAR && io->out_format != LWB_OUT_I16_PLANAR) return false;
     if (getenv("LWB_FORCE_GENERIC")) return false;
+    const bool itl_ok = long_takes_itl(io);
     for (auto &pc : plan) {
         const lwb_setup *su = pc.c->stream->setup;
         if (su->bs1 != kLongBs || !su->host.tab[1].pack) return false;
+        if (!long_step(io->out_format, su->channels, itl_ok)) return false;
         if (pc.c->status != LWB_OK) return false;
         for (auto &pp : pc.pk) {
             if (!pp.g.blockflag || pp.g.ls != 0 || pp.g.rs != (pp.g.n >> 1) || pp.g.re != pp.g.n) return false;
@@ -521,14 +560,15 @@ static int try_long_residue(lwb_ctx *ctx, lwb_chain *chains, size_t n_chains, co
     size_t n_sl = std::min<size_t>(std::max<size_t>(1, (n_pk * (size_t)C * kLongN2 * 4) >> 25), std::min<size_t>(8, n_chains));
     if (const char *e = getenv("LWB_E2E_CHUNKS")) n_sl = std::max<size_t>(1, std::min<size_t>((size_t)atol(e), std::min<size_t>(32, n_chains)));
     // whole-batch staging (absolute rows / offsets address it); each slice copies its own part
-    const size_t esz = io->out_format == LWB_OUT_I16_PLANAR ? 2 : 4;
+    const size_t esz = elem_size(io->out_format);
+    const bool planar = is_planar(io->out_format);
     uint64_t o_lo = ~0ull, o_hi = 0;
     for (size_t i = 0; i < n_chains; i++) {
         const lwb_chain *c = &chains[i];
         if (!c->n_packets) continue;
         const uint64_t ns = (uint64_t)(c->n_packets - (c->stream->has ? 0 : 1)) * kLongN2;
         o_lo = std::min(o_lo, c->out_offset);
-        o_hi = std::max(o_hi, c->out_offset + (uint64_t)(C - 1) * c->out_stride + ns);
+        o_hi = std::max(o_hi, pcm_end(c, C, planar, ns));
     }
     if (o_hi > o_lo && (rc = ensure(ctx, ctx->pcm, (size_t)(o_hi - o_lo) * esz))) return rc;
     const bool host_floors = io->floor_memory != LWB_MEM_DEVICE;
